@@ -9,11 +9,14 @@ A step = one ``SynthesizerTrn.infer`` over a batch of synthetic utterances (BASE
   roofline     : dominant kernel (tcgen05 ResBlock pair), CUDA-event device time inside this script
   cpu_baseline : the oracle port of the reference path on the host cores (bounded sample)
 ``--impl reference`` times that CPU port as the reference arm (the reference is pure Python/PyTorch; there is
-no compiled reference to build, and /root/reference does not exist on the GPU box).
+no compiled reference to build).
 ``--impl reference-cuda`` times the same reference ops as plain PyTorch on the B200 (cuDNN/ATen, TF32 default) - the
 denominator of BASELINE.json's ">= 5x the reference's PyTorch-CUDA infer" target.
 Other BASELINE configs: ``--vocoder nsf-snake-hifigan`` (config 4) and ``--workload flow5`` (config 5: flow-only
 microbench, z_p[1,192,100000]; reported in frames/s with the roofline in both FLOP and HBM units).
+``--dump-outputs DIR`` writes what the last timed step returned as ``DIR/<name>.npy`` (float32): ``audio`` and ``f0`` of
+``infer`` for config 2 / 4, ``z`` of the flow for config 5.  Weights, inputs and noise are seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -34,6 +37,7 @@ WORKLOAD_SNAKE = "config4: vdecoder/hifiganwithsnake Generator variant (nsf-snak
 WORKLOAD_FLOW5 = "config5: flow-only microbench, ResidualCouplingBlock WN stack 192ch x 4 flows, z_p[1,192,100000], g[1,768,1]"
 FLOW_FLOP_PER_FRAME = 14.156e6       # SURVEY §8d: 1 415.6 GFLOP at T = 100 000
 FLOW_BYTES_PER_FRAME_LAYER = 1152.0  # SURVEY §8d: per coupling layer, read 192 ch + write 96 ch fp32
+DUMP_BYTES = 60 << 20                # --dump-outputs: array data in all (< 64 MB with the .npy headers)
 
 
 def parse_args():
@@ -48,7 +52,27 @@ def parse_args():
     ap.add_argument("--batch", type=int, default=8, help="utterances per GPU")
     ap.add_argument("--frames", type=int, default=862)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of this project's path (--impl b200)")
+    return args
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Write each array as <out_dir>/<name>.npy in float32.  One larger than its share of DUMP_BYTES keeps a fixed, seeded
+    subset of its last (time) axis, in order, so that the dumps of two builds still compare element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[-1])
+            a = a[..., np.sort(np.random.default_rng(seed).choice(a.shape[-1], keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------- clocks
@@ -234,10 +258,10 @@ def run_flow5(args):
             flush.zero_()
         e[1].record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e[2].record()
         torch.cuda.synchronize()
-        return (e[1].elapsed_time(e[2]) - e[0].elapsed_time(e[1])) / steps
+        return (e[1].elapsed_time(e[2]) - e[0].elapsed_time(e[1])) / steps, last
 
     for _ in range(max(args.warmup, 3)):
         step_dev()
@@ -245,10 +269,12 @@ def run_flow5(args):
     sampler = ClockSampler(0)
     sampler.start()
     l0 = eng.launch_count
-    ms = timed(step_dev, args.steps)
+    ms, z_last = timed(step_dev, args.steps)
     launches = eng.launch_count - l0
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"z": z_last})
     peaks = {}
     pk_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(pk_path):
@@ -359,7 +385,7 @@ def main():
     d2h = out_host.numel() * out_host.element_size()
 
     def step_dev():
-        return net.infer(devin[0], devin[1], devin[2], g=devin[3], noice_scale=0.4)[0]
+        return net.infer(devin[0], devin[1], devin[2], g=devin[3], noice_scale=0.4)
 
     from sovits_b200.pipeline import HostPipeline
     pipe = HostPipeline(net, dev, depth=2)
@@ -389,7 +415,7 @@ def main():
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         barrier()
-        return float(ms.item())
+        return float(ms.item()), last
 
     # clocks are sampled from before the warm-up until after both timed regions (nvidia-smi needs ~0.2 s to produce its first
     # row; the timed regions are only ~0.1 s each), every 100 ms
@@ -406,9 +432,9 @@ def main():
         while not sampler.rows and time.time() - t_wait < 3.0:       # make sure the sampler is running before timing starts
             step_dev()
     l0 = eng.launch_count
-    ms_dev = timed(step_dev, args.steps)
+    ms_dev, (audio_last, f0_last) = timed(step_dev, args.steps)
     launches = (eng.launch_count - l0)
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     clocks = sampler.stop() if sampler else None
 
     # ---- roofline: CUDA events around every launch of each kernel family, on the launching stream (svb_profile_enable)
@@ -484,6 +510,16 @@ def main():
         cpu = {"value": rate, "unit": UNIT, "cores": cores, "kind": "port",
                "sample": f"oracle port of SynthesizerTrn.infer, the full batch ({B} utterances x {T} frames) once after a short "
                          f"warm-up ({sum(times):.1f} s of CPU work)"}
+
+    if args.dump_outputs:
+        outs = {"audio": audio_last, "f0": f0_last}
+        if world > 1:                          # every rank holds its block of the global batch
+            for k, t in outs.items():
+                parts = [torch.empty_like(t) for _ in range(world)]
+                dist.all_gather(parts, t.contiguous())
+                outs[k] = torch.cat(parts)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, outs)
 
     if rank == 0:
         total_samples = float(B * world * N)
